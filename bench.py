@@ -56,12 +56,20 @@ def parse_args():
     ap.add_argument('--cpu-steps', type=int, default=3)
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-e2e', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last one computed for rank 0 as DIR/<name>.npy: pos (lab-frame ligand '
+                         'positions, f32), v (atom types, f64), log_v0 / log_vt (the last v0_traj / vt_traj entry, f32); at most '
+                         '64 MB in all, beyond that a fixed seeded sample of ligand atoms, their indices in rows.npy')
     a = ap.parse_args()
     for k, v in WORKLOADS[a.workload].items():
         if getattr(a, k) is None:
             setattr(a, k, v)
     if a.full_chain:
         a.steps = CHAIN_STEPS
+    if not 1 <= a.steps <= CHAIN_STEPS:
+        ap.error('--steps must be in 1..%d: the timed steps are consecutive steps of one chain' % CHAIN_STEPS)
+    if a.dump_outputs and a.impl != 'ours':
+        ap.error('--dump-outputs writes the outputs of the GPU path (--impl ours)')
     return a
 
 
@@ -107,6 +115,26 @@ def measured_peaks():
         except Exception:
             pass
     return 6650.0, 'fallback (B200_PROFILING.md 6.65 TB/s)'
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write `arrays` (name -> host tensor with one row per ligand atom) as out_dir/<name>.npy in f32 / f64.  Above DUMP_LIMIT bytes
+    in all, the same seeded sample of rows goes into every file and the sampled row indices into rows.npy."""
+    import numpy as np
+    import torch
+    arrays = {k: v if v.is_floating_point() else v.double() for k, v in arrays.items()}      # class indices: exact in f64
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(v[0].numel() * v.element_size() for v in arrays.values())
+    if n * row_bytes > DUMP_LIMIT:
+        keep = (DUMP_LIMIT - 4096) // (row_bytes + 8)                                      # 8 bytes per index, npy headers
+        rows = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        arrays = dict({k: v[rows] for k, v in arrays.items()}, rows=rows.double())
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + '.npy'), v.numpy())
 
 
 class ClockSampler(threading.Thread):
@@ -319,6 +347,10 @@ def main():
     ms = ev0.elapsed_time(ev1)
     launches = lib.tdiff_launch_count(eng) - l0
     clocks = sampler.stop()
+    if a.dump_outputs and rank == 0:    # before the profiling chain below overwrites the trajectories
+        last = a.steps - 1
+        dump_outputs(a.dump_outputs, {'pos': traj[0][last].cpu(), 'v': traj[1][last].cpu(), 'log_v0': traj[2][last].cpu(),
+                                      'log_vt': traj[3][last].cpu()})
     if world > 1:
         t = torch.tensor([ms], device=dev, dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

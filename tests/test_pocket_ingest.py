@@ -1,4 +1,4 @@
-"""PDB pocket ingest + featurizer (SURVEY.md 8(f) n1).  The 1h36 check runs where the reference tree (its examples/) is present."""
+"""PDB pocket ingest + featurizer (SURVEY.md 8(f) n1)."""
 import os
 
 import numpy as np
@@ -48,12 +48,12 @@ def test_ligand_class_maps():
     assert is_aromatic_from_index(idx) == [False, False, True, False, True, False, True, False, False, True, False, True, False]
 
 
-REF_PDB = '/root/reference/examples/1h36_A_rec_1h36_r88_lig_tt_docked_0_pocket10.pdb'
+# the reference's examples/1h36_A_rec_1h36_r88_lig_tt_docked_0_pocket10.pdb, byte for byte
+PDB_1H36 = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', '1h36_pocket10.pdb')
 
 
-@pytest.mark.skipif(not os.path.exists(REF_PDB), reason='reference examples/ not present')
 def test_1h36_pocket_matches_survey_facts():
-    data = pdb_to_pocket_data(REF_PDB)
+    data = pdb_to_pocket_data(PDB_1H36)
     el = data.protein_element.tolist()
     assert len(el) == 572 and (el.count(6), el.count(7), el.count(8), el.count(16)) == (374, 87, 109, 2)      # SURVEY.md 8(c)
     assert len(set(data.protein_atom_to_aa_type.tolist())) == 19
