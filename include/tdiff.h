@@ -172,6 +172,47 @@ TDIFF_API int tdiff_scatter_mean3(const float* d_src, const int32_t* h_counts, i
 TDIFF_API int tdiff_check_stability(const float* d_pos, const int32_t* d_atomic_num, const int32_t* h_counts, int n_mol, int hs,
                                     int32_t* d_nr_bonds, int32_t* d_stable_atoms, uint8_t* d_mol_stable, void* stream);
 
+/* ---- binding-affinity regressor ---------------------------------------------------------------------------
+ * Replaces: PropPredNet / PropPredNetEnc with the EnEquiEncoder (models/property_pred/prop_model.py:27-165,
+ * models/property_pred/prop_egnn.py:8-83), inference only (scripts/property_prediction/inference.py).
+ * Kernels are built for hidden_dim 256, act_fn 'relu', norm False, edge_dim 0, num_r_gaussian 2..64, knn 1..64. */
+typedef struct tdiff_prop tdiff_prop;
+
+typedef struct tdiff_prop_config {
+  int32_t hidden_dim;        /* hidden_channels == encoder.hidden_dim, 256 (only value supported by the kernels) */
+  int32_t num_layers;        /* encoder.num_layers, >= 1 (6 in both published configs) */
+  int32_t knn;               /* encoder.knn, 1..64 (48) */
+  int32_t num_r_gaussian;    /* encoder.num_r_gaussian, 2..64 (64); centres come from encoder.distance_expansion.offset */
+  int32_t edge_dim;          /* encoder.edge_dim, must be 0 */
+  int32_t norm;              /* encoder.norm, must be 0 */
+  int32_t protein_feat_dim;  /* protein_atom_feature_dim (27) */
+  int32_t ligand_feat_dim;   /* ligand_atom_feature_dim: width of ligand_atom_feature_full, from the checkpoint */
+  int32_t enc_ligand_dim;    /* PropPredNetEnc: columns appended to the ligand features (0 for PropPredNet) */
+  int32_t enc_node_dim;      /* PropPredNetEnc: width of enc_node_feature; > 0 adds enc_node_layer */
+  int32_t enc_graph_dim;     /* PropPredNetEnc: columns appended to the pooled vector */
+  int32_t output_dim;        /* 3 (PropPredNet) or 1 (PropPredNetEnc) */
+  int32_t reserved[4];       /* must be 0 */
+} tdiff_prop_config;
+
+/* Copies and re-packs the weights (reference key names, fp32 host tensors; the per-layer r_expansion.offset buffers are
+ * accepted and ignored, as the reference never reads them).  Without a CUDA device: TDIFF_ECUDA. */
+TDIFF_API int tdiff_prop_create(const tdiff_prop_config* cfg, const tdiff_tensor* h_state_dict, int n_entries, int device, tdiff_prop** out);
+TDIFF_API void tdiff_prop_destroy(tdiff_prop* p);
+/* One forward.  h_protein_counts / h_ligand_counts: atoms per graph [n_graphs] (batch vectors sorted ascending).  Device inputs:
+ * d_protein_pos [Np,3], d_protein_feat [Np,protein_feat_dim], d_ligand_pos [Nl,3], d_ligand_feat [Nl,ligand_feat_dim] fp32;
+ * nullable like the reference's None: d_enc_ligand [Nl,enc_ligand_dim], d_enc_node [N,enc_node_dim] (composed node order: per graph,
+ * protein atoms then ligand atoms, = ScorePosNet3D.fetch_embedding's final_h order), d_enc_graph [n_graphs,enc_graph_dim],
+ * d_kind [n_graphs] int64 in 1..output_dim (output_kind; NULL returns every column).  Outputs: d_out [n_graphs,1] with d_kind,
+ * [n_graphs,output_dim] without; d_h_out [N,256] the encoder output in composed order (may be NULL).  Deterministic (no atomics).
+ * Synchronises the stream (a kind outside 1..output_dim is reported as TDIFF_EINVAL). */
+TDIFF_API int tdiff_prop_forward(tdiff_prop* p, int n_graphs, const int32_t* h_protein_counts, const int32_t* h_ligand_counts,
+                                 const float* d_protein_pos, const float* d_protein_feat, const float* d_ligand_pos, const float* d_ligand_feat,
+                                 const float* d_enc_ligand, const float* d_enc_node, const float* d_enc_graph, const int64_t* d_kind,
+                                 float* d_out, float* d_h_out, void* stream);
+/* Time (ms, CUDA events) and count of the encoder edge-kernel launches accumulated while profiling is on (enable != 0 resets). */
+TDIFF_API int tdiff_prop_profile(tdiff_prop* p, int enable);
+TDIFF_API int tdiff_prop_profile_read(tdiff_prop* p, double* ms_edge, int64_t* n_edge_launches, int64_t* n_edge_rows);
+
 /* ---- instrumentation ------------------------------------------------------------------------------------
  * Number of kernel launches issued by this engine since creation (graph replays count their nodes). */
 TDIFF_API int64_t tdiff_launch_count(tdiff_engine* e);

@@ -25,6 +25,13 @@ class tdiff_config(ctypes.Structure):
                 ('reserved', ctypes.c_int32 * 2)]
 
 
+class tdiff_prop_config(ctypes.Structure):
+    _fields_ = [('hidden_dim', ctypes.c_int32), ('num_layers', ctypes.c_int32), ('knn', ctypes.c_int32), ('num_r_gaussian', ctypes.c_int32),
+                ('edge_dim', ctypes.c_int32), ('norm', ctypes.c_int32), ('protein_feat_dim', ctypes.c_int32), ('ligand_feat_dim', ctypes.c_int32),
+                ('enc_ligand_dim', ctypes.c_int32), ('enc_node_dim', ctypes.c_int32), ('enc_graph_dim', ctypes.c_int32),
+                ('output_dim', ctypes.c_int32), ('reserved', ctypes.c_int32 * 4)]
+
+
 class tdiff_tensor(ctypes.Structure):
     _fields_ = [('name', ctypes.c_char_p), ('data', ctypes.c_void_p), ('numel', ctypes.c_int64)]
 
@@ -55,6 +62,11 @@ SIGNATURES = {
     'tdiff_attn_aggregate_x': (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _vp]),
     'tdiff_scatter_mean3': (_i, [_vp, _pi32, _i, _vp, _vp]),
     'tdiff_check_stability': (_i, [_vp, _vp, _pi32, _i, _i, _vp, _vp, _vp, _vp]),
+    'tdiff_prop_create': (_i, [ctypes.POINTER(tdiff_prop_config), ctypes.POINTER(tdiff_tensor), _i, _i, ctypes.POINTER(_vp)]),
+    'tdiff_prop_destroy': (None, [_vp]),
+    'tdiff_prop_forward': (_i, [_vp, _i, _pi32, _pi32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    'tdiff_prop_profile': (_i, [_vp, _i]),
+    'tdiff_prop_profile_read': (_i, [_vp, ctypes.POINTER(ctypes.c_double), ctypes.POINTER(_i64), ctypes.POINTER(_i64)]),
     'tdiff_launch_count': (_i64, [_vp]),
     'tdiff_edge_mlp_mode': (_i, [_vp]),
     'tdiff_profile': (_i, [_vp, _i]),

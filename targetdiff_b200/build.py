@@ -17,7 +17,7 @@ CSRC = os.path.join(HERE, 'csrc')
 _VARIANT = os.environ.get('TDIFF_VARIANT', '')
 OBJ = os.path.join(CSRC, 'build' + ('_' + _VARIANT if _VARIANT else ''))
 LIB = os.path.join(HERE, 'libtdiff%s.so' % ('_' + _VARIANT if _VARIANT else ''))
-SOURCES = ['engine.cu', 'knn.cu', 'edge_const.cu', 'node_ops.cu', 'edge_mlp.cu', 'edge_mlp_tc.cu', 'edge_mlp_v4.cu', 'aggregate.cu', 'sampler.cu', 'stability.cu']
+SOURCES = ['engine.cu', 'knn.cu', 'edge_const.cu', 'node_ops.cu', 'edge_mlp.cu', 'edge_mlp_tc.cu', 'edge_mlp_v4.cu', 'aggregate.cu', 'sampler.cu', 'stability.cu', 'prop.cu']
 HEADERS = ['tdiff_common.cuh', 'sampler.cuh', os.path.join('..', '..', 'include', 'tdiff.h')]
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-O3', '-lineinfo', '-std=c++17', '-Xcompiler', '-fPIC',
               '-Xcompiler', '-fvisibility=hidden', '-Xptxas', '-v']

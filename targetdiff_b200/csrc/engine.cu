@@ -31,6 +31,14 @@ static int set_err(int code, const char* fmt, ...) {
   va_end(ap);
   return code;
 }
+// the same error slot for the entry points defined in other translation units (prop.cu)
+int td_set_err(int code, const char* fmt, ...) {
+  va_list ap;
+  va_start(ap, fmt);
+  vsnprintf(g_err, sizeof(g_err), fmt, ap);
+  va_end(ap);
+  return code;
+}
 #define CK(call)                                                                                       \
   do {                                                                                                 \
     cudaError_t _e = (call);                                                                           \

@@ -140,6 +140,9 @@ inline void td_opt_in_smem(Kernel kernel, size_t bytes, size_t (&done)[TD_MAX_DE
   if (known) done[dev] = bytes;
 }
 
+// tdiff_last_error() text for entry points outside engine.cu; returns `code`
+int td_set_err(int code, const char* fmt, ...);
+
 // Launchers (defined in the .cu files, called by engine.cu).  All asynchronous on `st`.
 // `stride` = slots per row (>= k); `hybrid` != 0: ligand rows = other ligand atoms + k nearest protein atoms (prot_ptr required)
 void td_launch_knn(const float4* xm, const int* node_ptr, const int* prot_ptr, int n_graphs, int max_nodes_per_graph, int k, int stride, int hybrid,
