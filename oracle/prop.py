@@ -37,8 +37,9 @@ def _lin(key, out_dim, in_dim):
     return [(key + '.weight', (out_dim, in_dim), 'lin_w'), (key + '.bias', (out_dim,), 'lin_b:%d' % in_dim)]
 
 
-def state_dict_spec(config, protein_dim=PROTEIN_FEATURE_DIM, ligand_dim=LIGAND_FEATURE_DIM):
-    """Ordered (key, shape, kind) list == the reference module's state_dict() (prop_model.py:29-45,99-128, prop_egnn.py:8-26,49-72)."""
+def state_dict_spec(config, protein_dim=PROTEIN_FEATURE_DIM, ligand_dim=LIGAND_FEATURE_DIM, output_dim=None):
+    """Ordered (key, shape, kind) list == the reference module's state_dict() (prop_model.py:29-45,99-128, prop_egnn.py:8-26,49-72).
+    output_dim None: the reference's get_model choice (3 for PropPredNet, 1 for PropPredNetEnc)."""
     enc = config['encoder']
     H, G, L = config['hidden_channels'], enc['num_r_gaussian'], enc['num_layers']
     is_enc = enc['name'] == 'egnn_enc'
@@ -55,15 +56,17 @@ def state_dict_spec(config, protein_dim=PROTEIN_FEATURE_DIM, ligand_dim=LIGAND_F
     if is_enc and config.get('enc_node_dim', 0) > 0:
         spec += _lin('enc_node_layer.0', H, H + config['enc_node_dim']) + _lin('enc_node_layer.2', H, H)
     gdim = config.get('enc_graph_dim', 0) if is_enc else 0
-    spec += _lin('out_block.0', H, H + gdim) + _lin('out_block.2', 1 if is_enc else 3, H)
+    if output_dim is None:
+        output_dim = 1 if is_enc else 3
+    spec += _lin('out_block.0', H, H + gdim) + _lin('out_block.2', output_dim, H)
     return spec
 
 
-def make_state_dict(config, seed=0, gain=1.0, protein_dim=PROTEIN_FEATURE_DIM, ligand_dim=LIGAND_FEATURE_DIM):
+def make_state_dict(config, seed=0, gain=1.0, protein_dim=PROTEIN_FEATURE_DIM, ligand_dim=LIGAND_FEATURE_DIM, output_dim=None):
     """Deterministic weights, Linear: U(-1/sqrt(in), 1/sqrt(in)) * gain (nn.Linear's default bound), like oracle.synth."""
     g = torch.Generator().manual_seed(seed)
     sd = {}
-    for key, shape, kind in state_dict_spec(config, protein_dim, ligand_dim):
+    for key, shape, kind in state_dict_spec(config, protein_dim, ligand_dim, output_dim):
         if kind.startswith('offset'):
             sd[key] = torch.linspace(0.0, float(kind.split(':')[1]), shape[0])              # GaussianSmearing(fixed_offset=False)
         elif kind == 'lin_w':
@@ -87,57 +90,150 @@ def compose_stable(batch_protein, batch_ligand):
     return torch.sort(torch.cat([batch_protein, batch_ligand]), stable=True).indices
 
 
-def _linear_relu_linear(sd, prefix, x, act=F.relu, i0=0, i1=2):
-    y = act(F.linear(x, sd['%s.%d.weight' % (prefix, i0)], sd['%s.%d.bias' % (prefix, i0)]))
-    return F.linear(y, sd['%s.%d.weight' % (prefix, i1)], sd['%s.%d.bias' % (prefix, i1)])
+def plain_linear(key, x, w, b):
+    """The default `linear` hook: F.linear.  `key` is the state_dict key of the weight (which Linear this is)."""
+    return F.linear(x, w, b)
+
+
+def _apply(linear, sd, prefix, x):
+    return linear(prefix + '.weight', x, sd[prefix + '.weight'], sd[prefix + '.bias'])
+
+
+def _linear_relu_linear(sd, prefix, x, act=F.relu, i0=0, i1=2, linear=plain_linear):
+    y = act(_apply(linear, sd, '%s.%d' % (prefix, i0), x))
+    return _apply(linear, sd, '%s.%d' % (prefix, i1), y)
 
 
 def shifted_softplus(x):
     return F.softplus(x) - torch.log(torch.tensor(2.0)).item()                               # models/common.py:156-162
 
 
-def encoder_forward(sd, enc, h, pos, batch, trace=None):
-    """EnEquiEncoder.forward (prop_egnn.py:74-83), update_x=False, norm=False, act_fn='relu'."""
+def encoder_forward(sd, enc, h, pos, batch, trace=None, linear=plain_linear):
+    """EnEquiEncoder.forward (prop_egnn.py:74-83), update_x=False, norm=False, act_fn='relu'.  The edge set comes from the fp32
+    positions (knn_graph_canonical casts); the edge lengths from `pos` as given, so a float64 run widens the fp32 values."""
     ei = knn_graph_canonical(pos, enc['knn'], batch)          # rows (src, dst) == knn_graph(flow='target_to_source') unpacked dst, src
     src, dst = ei[0], ei[1]
     edge_length = torch.norm(pos[dst] - pos[src], dim=1)                                      # :79
     edge_attr = gaussian_smearing(edge_length, sd['encoder.distance_expansion.offset'])      # :80, common.py:7-26
     for l in range(enc['num_layers']):                                                        # :82-83
         p = 'encoder.net.%d' % l
-        m = F.relu(_linear_relu_linear(sd, p + '.edge_mlp.net', torch.cat([edge_attr, h[dst], h[src]], -1)))   # :34-35 (act_last=True)
-        e = torch.sigmoid(F.linear(m, sd[p + '.edge_inf.0.weight'], sd[p + '.edge_inf.0.bias']))              # :36
+        m = F.relu(_linear_relu_linear(sd, p + '.edge_mlp.net', torch.cat([edge_attr, h[dst], h[src]], -1), linear=linear))   # :34-35
+        e = torch.sigmoid(_apply(linear, sd, p + '.edge_inf.0', m))                                                    # :36
         mi = torch.zeros_like(h).index_add_(0, dst, m * e)                                                     # :37 scatter_sum
-        h = h + _linear_relu_linear(sd, p + '.node_mlp.net', torch.cat([mi, h], -1))                         # :41, :83
+        h = h + _linear_relu_linear(sd, p + '.node_mlp.net', torch.cat([mi, h], -1), linear=linear)          # :41, :83
     if trace is not None:
         trace['edge_index'] = ei
     return h
 
 
 def prop_forward(sd, config, protein_pos, protein_feat, ligand_pos, ligand_feat, batch_protein, batch_ligand, output_kind=None,
-                 enc_ligand=None, enc_node=None, enc_graph=None, trace=None):
-    """PropPredNet.forward (prop_model.py:48-74) / PropPredNetEnc.forward (:130-165).  `enc_node` is in the stable composed order."""
+                 enc_ligand=None, enc_node=None, enc_graph=None, trace=None, linear=plain_linear):
+    """PropPredNet.forward (prop_model.py:48-74) / PropPredNetEnc.forward (:130-165).  `enc_node` is in the stable composed order.
+    `linear(key, x, w, b)` computes every Linear (key: the state_dict key of its weight); see tensor_core_linear."""
     enc = config['encoder']
     if enc_ligand is not None:
         ligand_feat = torch.cat([ligand_feat, enc_ligand], -1)                                 # :133-134
-    h_p = F.linear(protein_feat, sd['protein_atom_emb.weight'], sd['protein_atom_emb.bias'])
-    h_l = F.linear(ligand_feat, sd['ligand_atom_emb.weight'], sd['ligand_atom_emb.bias'])
+    h_p = _apply(linear, sd, 'protein_atom_emb', protein_feat)
+    h_l = _apply(linear, sd, 'ligand_atom_emb', ligand_feat)
     order = compose_stable(batch_protein, batch_ligand)                                       # common.py:140-153
     h = torch.cat([h_p, h_l])[order]
     pos = torch.cat([protein_pos, ligand_pos])[order]
     batch = torch.cat([batch_protein, batch_ligand])[order]
-    h = encoder_forward(sd, enc, h, pos, batch, trace)
+    h = encoder_forward(sd, enc, h, pos, batch, trace, linear)
     if trace is not None:
         trace['h'] = h
     if enc_node is not None:                                                                  # :146-148
-        h = _linear_relu_linear(sd, 'enc_node_layer', torch.cat([h, enc_node], -1))
+        h = _linear_relu_linear(sd, 'enc_node_layer', torch.cat([h, enc_node], -1), linear=linear)
     n_graphs = int(max(batch_protein.max().item() if len(batch_protein) else -1, batch_ligand.max().item() if len(batch_ligand) else -1)) + 1
-    pre = torch.zeros(n_graphs, h.shape[1]).index_add_(0, batch, h)                            # :151 scatter sum
+    pre = torch.zeros(n_graphs, h.shape[1], dtype=h.dtype).index_add_(0, batch, h)                            # :151 scatter sum
     if enc_graph is not None:
         pre = torch.cat([pre, enc_graph], -1)                                                 # :152-153
-    out = _linear_relu_linear(sd, 'out_block', pre, act=shifted_softplus)                     # :155
+    out = _linear_relu_linear(sd, 'out_block', pre, act=shifted_softplus, linear=linear)      # :155
     if output_kind is not None:                                                               # :156-158
         out = torch.sum(out * F.one_hot(output_kind - 1, out.shape[1]), dim=-1, keepdim=True)
     return out
+
+
+# ----------------------------------------------------------------------------------------------------- bf16-split emulation
+# csrc/prop.cu runs every Linear below on tcgen05 in the two-piece bf16 split; edge_inf.0 (gate) and out_block run as fp32 FMA on
+# CUDA cores.  edge_mlp.net.0 is one product over all G + 512 input columns: the kernels' gaussian / h_dst / h_src blocks sum to it.
+TENSOR_CORE_LINEARS = ('protein_atom_emb', 'ligand_atom_emb', 'edge_mlp.net.0', 'edge_mlp.net.2', 'node_mlp.net.0', 'node_mlp.net.2',
+                       'enc_node_layer.0', 'enc_node_layer.2')
+
+
+def bf16_split(t):
+    """fp32 t -> (t1, t2) in float64: t1 = bf16_rn(t), t2 = bf16_rn(t - t1) (t - t1 is exact in fp32)."""
+    t = t.to(torch.float32)
+    t1 = t.to(torch.bfloat16).to(torch.float32)
+    t2 = (t - t1).to(torch.bfloat16).to(torch.float32)
+    return t1.double(), t2.double()
+
+
+def split_linear(x, w, b=None):
+    """prop_gemm_kernel / prop_edge_kernel arithmetic: both operands rounded to fp32 and split, y = x1.w1^T + x1.w2^T + x2.w1^T
+    accumulated in float64 (the kernels accumulate in fp32), then the fp32 bias.  |y - x.w^T| <= ~3 * 2^-16 * |x|.|w|^T."""
+    x1, x2 = bf16_split(x)
+    w1, w2 = bf16_split(w)
+    y = x1 @ w1.T + x1 @ w2.T + x2 @ w1.T
+    return y if b is None else y + b.to(torch.float32).double()
+
+
+def tensor_core_linear(key, x, w, b):
+    """`linear` hook of prop_forward that emulates the split on the Linears that run on tensor cores, plain F.linear elsewhere."""
+    name = key[:-len('.weight')]
+    if any(name == t or name.endswith('.' + t) for t in TENSOR_CORE_LINEARS):
+        return split_linear(x, w, b)
+    return F.linear(x, w, b)
+
+
+def to_float64(sd_or_inputs):
+    """float tensors of a state_dict / an input dict widened to float64 (integer tensors and None unchanged)."""
+    return {k: (v.double() if torch.is_tensor(v) and v.is_floating_point() else v) for k, v in sd_or_inputs.items()}
+
+
+def forward_float64(sd, config, x, linear=plain_linear, trace=None):
+    """prop_forward on the float64 widening of `sd` and the input dict `x` (pin_inputs keys)."""
+    sd, x = to_float64(sd), to_float64(x)
+    return prop_forward(sd, config, x['protein_pos'], x['protein_feat'], x['ligand_pos'], x['ligand_feat'], x['batch_protein'],
+                        x['batch_ligand'], x['output_kind'], x['enc_ligand'], x['enc_node'], x['enc_graph'], trace=trace, linear=linear)
+
+
+def emulate_split(sd, config, x, trace=None):
+    """What the B200 kernels compute, up to their fp32 accumulation: float64 everywhere, bf16 split on the tensor-core Linears."""
+    return forward_float64(sd, config, x, linear=tensor_core_linear, trace=trace)
+
+
+def forward_with_gates(sd, config, x, linear=plain_linear, gate_override=None):
+    """forward_float64 that also returns every layer's edge-gate logits (edge_inf.0 outputs, edge order of trace['edge_index']).
+    gate_override {layer: (edge indices, logits)} replaces those logits before the sigmoid.  Returns (pred, h, [logits per layer])."""
+    gates, tr = [], {}
+
+    def hooked(key, xx, w, b):
+        y = linear(key, xx, w, b)
+        if key.endswith('.edge_inf.0.weight'):
+            if gate_override and len(gates) in gate_override:
+                idx, z = gate_override[len(gates)]
+                y = y.clone()
+                y[idx, 0] = z.to(y.dtype)
+            gates.append(y[:, 0])
+        return y
+    out = forward_float64(sd, config, x, linear=hooked, trace=tr)
+    return out, tr['h'], gates, tr['edge_index']
+
+
+def gate_flips(sd, config, x):
+    """Edges whose gate the split's own error switches: sigmoid(logit) differs by more than 1/2 between the float64 forward and
+    emulate_split.  With large weights the logits reach ~1e8 and the sigmoid is a step, so a logit within the split's error of 0 decides
+    whether a whole message enters its destination's sum: a knife edge, not a kernel defect.  Returns {layer: edge indices} and the
+    float64 logits, so forward_with_gates(..., gate_override=...) can put the emulation on the float64 side of every flipped gate."""
+    _, _, z64, ei = forward_with_gates(sd, config, x)
+    _, _, zemu, _ = forward_with_gates(sd, config, x, linear=tensor_core_linear)
+    flips = {}
+    for l, (a, b) in enumerate(zip(z64, zemu)):
+        idx = torch.nonzero((torch.sigmoid(a) - torch.sigmoid(b)).abs() > 0.5).flatten()
+        if len(idx):
+            flips[l] = idx
+    return flips, z64, ei
 
 
 # ----------------------------------------------------------------------------------------------------- reference pins

@@ -104,33 +104,51 @@ def test_two_calls_bit_identical():
 
 
 def test_alone_equals_inside_ragged_batch():
-    """Per-destination padding of the edge tile: a complex's result does not depend on its neighbours in the batch (bit-identical)."""
+    """Per-destination padding of the edge tile: a complex's result does not depend on its neighbours in the batch (bit-identical),
+    for every graph of a 66-graph ragged batch that includes an empty graph (pooled to 0) followed by a graph with an odd atom count."""
     config = prop.EGNN_CONFIG
     model, _ = _model(config, 0)
     rng = np.random.RandomState(5)
     psizes = [int(v) for v in rng.randint(20, 400, size=64)]
     lsizes = [int(v) for v in rng.randint(5, 40, size=64)]
+    empty = 30
+    psizes[empty:empty] = [0, 37]
+    lsizes[empty:empty] = [0, 8]
+    B = len(psizes)
     ppos, pfeat, lpos = [], [], []
     g = torch.Generator().manual_seed(11)
     for i, (npr, nl) in enumerate(zip(psizes, lsizes)):
+        if npr == 0:
+            ppos.append(torch.zeros(0, 3)), pfeat.append(torch.zeros(0, synth.PROTEIN_FEATURE_DIM)), lpos.append(torch.zeros(0, 3))
+            continue
         p, f = synth.make_pocket(500 + i, npr)
         ppos.append(p), pfeat.append(f)
         lpos.append(p.mean(0, keepdim=True) + torch.randn(nl, 3, generator=g))
     lfeat = prop.make_ligand_features(9, sum(lsizes))
-    bp = torch.repeat_interleave(torch.arange(64), torch.tensor(psizes))
-    bl = torch.repeat_interleave(torch.arange(64), torch.tensor(lsizes))
+    bp = torch.repeat_interleave(torch.arange(B), torch.tensor(psizes))
+    bl = torch.repeat_interleave(torch.arange(B), torch.tensor(lsizes))
     x = dict(protein_pos=torch.cat(ppos), protein_feat=torch.cat(pfeat), ligand_pos=torch.cat(lpos), ligand_feat=lfeat, batch_protein=bp,
              batch_ligand=bl, output_kind=None, enc_ligand=None, enc_node=None, enc_graph=None)
     full, hfull = _run(model, config, x)
-    j = 37
-    pstart, lstart = sum(psizes[:j]), sum(lsizes[:j])
-    one = dict(protein_pos=ppos[j], protein_feat=pfeat[j], ligand_pos=lpos[j], ligand_feat=lfeat[lstart:lstart + lsizes[j]],
-               batch_protein=torch.zeros(psizes[j], dtype=torch.long), batch_ligand=torch.zeros(lsizes[j], dtype=torch.long), output_kind=None,
-               enc_ligand=None, enc_node=None, enc_graph=None)
-    alone, halone = _run(model, config, one)
-    n0 = pstart + lstart
-    assert torch.equal(alone[0], full[j])
-    assert torch.equal(halone, hfull[n0:n0 + psizes[j] + lsizes[j]])
+
+    def sub(graphs):
+        p0, l0 = sum(psizes[:graphs[0]]), sum(lsizes[:graphs[0]])
+        ps, ls = [psizes[j] for j in graphs], [lsizes[j] for j in graphs]
+        return dict(protein_pos=torch.cat([ppos[j] for j in graphs]), protein_feat=torch.cat([pfeat[j] for j in graphs]),
+                    ligand_pos=torch.cat([lpos[j] for j in graphs]), ligand_feat=lfeat[l0:l0 + sum(ls)],
+                    batch_protein=torch.repeat_interleave(torch.arange(len(graphs)), torch.tensor(ps)),
+                    batch_ligand=torch.repeat_interleave(torch.arange(len(graphs)), torch.tensor(ls)), output_kind=None,
+                    enc_ligand=None, enc_node=None, enc_graph=None), p0 + l0
+    for j in range(B):
+        if j == empty:          # a batch of one empty graph is rejected: score it together with its odd-sized neighbour
+            one, n0 = sub([j, j + 1])
+        elif j == empty + 1:
+            continue
+        else:
+            one, n0 = sub([j])
+        alone, halone = _run(model, config, one)
+        assert torch.equal(alone, full[j:j + len(alone)]), j
+        assert torch.equal(halone, hfull[n0:n0 + len(halone)]), j
 
 
 def test_fetch_embedding_final_h_chain():

@@ -92,6 +92,17 @@ def precision_on_pins(dev):
             r = dict(pred_max_abs_err_vs_oracle=(out - want).abs().max().item(),
                      pred_max_rel_err_vs_oracle=((out - want).abs() / want.abs().clamp_min(1e-30)).max().item(),
                      h_max_err_over_max_abs_h_vs_oracle=(h - tr['h']).abs().max().item() / tr['h'].abs().max().item())
+            # against the float64 emulation of the kernels' bf16 split; where the split's error switches an edge gate (a logit
+            # within that error of 0), also against the emulation with those gates on the float64 side
+            flips, z64, ei = prop.gate_flips(sd, config, x)
+            sides = {'split_emulation': None}
+            if flips:
+                sides['split_emulation_fp64_gates'] = {l: (i, z64[l][i]) for l, i in flips.items()}
+            for label, ov in sides.items():
+                eo, eh, _, _ = prop.forward_with_gates(sd, config, x, linear=prop.tensor_core_linear, gate_override=ov)
+                r['h_max_err_over_max_abs_h_vs_' + label] = (h.double() - eh).abs().max().item() / eh.abs().max().item()
+                r['pred_max_err_over_max_abs_pred_vs_' + label] = (out.double() - eo).abs().max().item() / max(eo.abs().max().item(), 1.0)
+            r['gate_flips_layer_src_dst'] = [(l, ei[0, i].item(), ei[1, i].item()) for l, idx in flips.items() for i in idx]
             if gain == 1.0:
                 ref = torch.from_numpy(pins[name + '__pred'])
                 hr = torch.from_numpy(pins[name + '__h'])
